@@ -128,6 +128,18 @@ def engine_config(cfg, gemm_mode, lm=None):
     return ec
 
 
+def dump_outputs(out_dir, out):
+    """Writes what the headline path returned for its last timed batch as <out_dir>/<name>.npy (float64; token slots past
+    a row's ntok are -1, so two builds compare equal when they emit the same transcripts)."""
+    os.makedirs(out_dir, exist_ok=True)
+    tokens = out["tokens"].cpu().numpy().astype(np.float64)
+    ntok = out["ntok"].cpu().numpy()
+    tokens[np.arange(tokens.shape[1])[None, :] >= ntok[:, None]] = -1.0
+    arrays = {"tokens": tokens, "ntok": ntok.astype(np.float64), "neg_logp": out["neg_logp"].cpu().numpy().astype(np.float64)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def timed_ms(fn, steps, warmup, dev):
     for _ in range(warmup):
         fn()
@@ -346,6 +358,8 @@ def run_product(args):
     evals, emitted = int(iters.sum()), int(sum(len(t) for t in toks))
 
     if args.profile:
+        if rank == 0 and args.dump_outputs:
+            dump_outputs(args.dump_outputs, res)
         if rank == 0:
             print(json.dumps({"profile_run": True, "ms_per_step": ms_total / args.steps, "launches_per_step": int(launches),
                               "stage_ms": stage}), flush=True)
@@ -405,6 +419,8 @@ def run_product(args):
         if pipe_ms_total < ms_total:
             ms_total, pipe_depth = pipe_ms_total, 2
         _trace(f"pipelined loop done: {pipe_ms_total / args.steps:.3f} vs {seq_ms_total / args.steps:.3f} ms per step")
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, last if pipe_depth == 2 else res)
 
     # ---- end-to-end through the public host-buffer call (e2e) ----
     def gather_tokens(o=None):
@@ -672,7 +688,13 @@ def main():
     ap.add_argument("--profile", action="store_true",
                     help="for runs under ncu: device-resident steps only, no e2e / CPU legs, warm-up not forced to 3 "
                          "(numbers printed in this mode are not bench values)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the headline path's outputs for its last batch as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
     if not args.profile:
         args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
