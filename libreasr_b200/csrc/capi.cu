@@ -307,7 +307,7 @@ int32_t rnnt_b200_create(const rnnt_b200_config* cfg, rnnt_b200_handle* out) {
   h = new rnnt_b200_handle_s();
   h->cfg = *cfg;
   h->sm_count = prop.multiProcessorCount;
-  if ((e = configure_lstm()) != cudaSuccess || (e = configure_gemm_tc()) != cudaSuccess || (e = configure_gemm_tc2()) != cudaSuccess ||
+  if ((e = configure_lstm()) != cudaSuccess || (e = configure_gemm_tc()) != cudaSuccess ||
       (e = configure_lstm_tc()) != cudaSuccess || (e = configure_lstm_tc2()) != cudaSuccess || (e = configure_decode_tc()) != cudaSuccess || (e = configure_decode_tc2()) != cudaSuccess || (e = configure_decode(cfg->device, &h->coop_blocks)) != cudaSuccess) {
     delete h;
     return fail_cuda(nullptr, e, "kernel configuration");
@@ -912,6 +912,74 @@ int32_t rnnt_b200_resample(rnnt_b200_handle h, const float* audio, int32_t B, in
   return RNNT_B200_OK;
 }
 
+// Recurrent kernels of the encoder and the decode loop: the fp32 kernels (lstm.cu / decode.cu), the round-1 persistent
+// tcgen05 kernels (lstm_tc.cu / decode_tc.cu) and the cluster split-K kernels (lstm_tc2.cu / decode_tc2.cu).
+enum class RecKernel { Fp32, Tc, Tc2 };
+
+struct EncoderRoute {
+  RecKernel kernel;
+  int rows;          // rows per launch: a call with more rows runs as consecutive sub-batches
+  LstmTcPlan tc;     // plan of a launch of `rows` rows (kernel Tc)
+  LstmTc2Plan tc2;   // ... (kernel Tc2)
+};
+
+// The encoder's kernel for a call of B rows.  Stateless batches beyond 32 rows run as 32-row sub-batches of the cluster
+// kernel (measured on a B200: 64 utterances 50.0k x real time vs 44.6k in one 64-row launch of the round-1 kernel, 256
+// utterances equal); streaming ticks (T = 2, carried state) are faster in one wide launch of the round-1 kernel (8.7k vs 8.0k x).
+static EncoderRoute route_encoder(rnnt_b200_handle h, int B, bool stateful) {
+  EncoderRoute r = {};
+  r.kernel = RecKernel::Fp32;
+  r.rows = B;
+  if (h->cfg.gemm_mode != RNNT_B200_GEMM_TC_FP16X3) return r;
+  const int H = h->cfg.hidden_sz;
+  const int cap = (!stateful && h->lstm_tc2_ok) ? 32 : 128;
+  if (h->lstm_tc_ok && B > cap) r.rows = cap;   // (without the round-1 kernel a call is never split: one launch of the fp32 kernel)
+  if (h->lstm_tc2_ok && lstm_tc2_plan(H, r.rows, h->sm_count, &r.tc2)) r.kernel = RecKernel::Tc2;
+  else if (h->lstm_tc_ok && lstm_tc_plan(H, r.rows, h->sm_count, &r.tc)) r.kernel = RecKernel::Tc;
+  return r;
+}
+
+// RNNT_LSTM_DBG: per-step phase times of CTA 0, the publish skew over all CTAs and CTA 0's cycle breakdown of one
+// cluster-kernel layer, on stderr (tuning aid: synchronises the stream; frees the stamp buffers)
+static int32_t report_lstm_stamps(rnnt_b200_handle h, const LstmTc2Args& a, int grid, cudaStream_t st) {
+  const int B = a.B, T = a.T;
+  std::vector<unsigned long long> ha((size_t)grid * T * 2), hb((size_t)T * 4 + 16);
+  CK(cudaStreamSynchronize(st));
+  CK(cudaMemcpy(ha.data(), a.dbg_all, ha.size() * 8, cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy(hb.data(), a.dbg, (size_t)T * 32 + 128, cudaMemcpyDeviceToHost));
+  cudaFree(a.dbg_all);
+  cudaFree(a.dbg);
+  double sp_pub = 0, sp_red = 0, first_to_last = 0;
+  for (int t = 1; t < T; ++t) {
+    unsigned long long mn = ~0ull, mx = 0, mn2 = ~0ull, mx2 = 0;
+    for (int c2 = 0; c2 < grid; ++c2) {
+      const unsigned long long a0 = ha[((size_t)c2 * T + t) * 2], a1 = ha[((size_t)c2 * T + t) * 2 + 1];
+      mn = std::min(mn, a0); mx = std::max(mx, a0); mn2 = std::min(mn2, a1); mx2 = std::max(mx2, a1);
+    }
+    sp_pub += (double)(mx - mn); sp_red += (double)(mx2 - mn2);
+    unsigned long long pm = 0;
+    for (int c2 = 0; c2 < grid; ++c2) pm = std::max(pm, ha[((size_t)c2 * T + t - 1) * 2]);
+    first_to_last += (double)(mn2 - pm);   // last publish of step t-1 -> first CTA with complete tiles at step t
+  }
+  fprintf(stderr, "[lstm_tc2 skew] avg ns over %d CTAs: spread of publish times %.0f | spread of tiles-complete times %.0f | last publish(t-1) -> first tiles-complete(t) %.0f\n",
+          grid, sp_pub / (T - 1), sp_red / (T - 1), first_to_last / (T - 1));
+  fprintf(stderr, "[lstm_tc2 epilogue cycles/step, CTA 0 thread 0] wait accumulators %.0f | TMEM drain %.0f | scatter issue %.0f | wait tiles %.0f | tile sums %.0f | cell %.0f | publish %.0f | BN outputs %.0f\n",
+          (double)hb[(size_t)T * 4 + 0] / T, (double)hb[(size_t)T * 4 + 1] / T, (double)hb[(size_t)T * 4 + 2] / T, (double)hb[(size_t)T * 4 + 3] / T,
+          (double)hb[(size_t)T * 4 + 4] / T, (double)hb[(size_t)T * 4 + 5] / T, (double)hb[(size_t)T * 4 + 6] / T, (double)hb[(size_t)T * 4 + 7] / T);
+  fprintf(stderr, "[lstm_tc2 loader cycles/step, CTA 0 thread 0] first chunk visible %.0f | k-block 0 valid %.0f | k-blocks 1-3 valid %.0f | stores+fence+arrive %.0f\n",
+          (double)hb[(size_t)T * 4 + 8] / T, (double)hb[(size_t)T * 4 + 9] / T, (double)hb[(size_t)T * 4 + 10] / T, (double)hb[(size_t)T * 4 + 11] / T);
+  double ld = 0, mma = 0, red = 0, fin = 0;
+  for (int t = 1; t < T; ++t) {
+    ld += (double)(hb[t * 4 + 0] - hb[(t - 1) * 4 + 3]);   // previous publish -> K slice of h landed in smem
+    mma += (double)(hb[t * 4 + 1] - hb[t * 4 + 0]);        // -> accumulators ready
+    red += (double)(hb[t * 4 + 2] - hb[t * 4 + 1]);        // TMEM drain + DSMEM scatter + partial tiles complete
+    fin += (double)(hb[t * 4 + 3] - hb[t * 4 + 2]);        // cell + publish
+  }
+  fprintf(stderr, "[lstm_tc2 dbg] B=%d T=%d steps avg ns: publish->h landed %.0f | ->tmem_full %.0f | drain+reduce %.0f | cell+publish %.0f | total/step %.0f\n",
+          B, T, ld / (T - 1), mma / (T - 1), red / (T - 1), fin / (T - 1), (double)(hb[(T - 1) * 4 + 3] - hb[3]) / (T - 1));
+  return RNNT_B200_OK;
+}
+
 static int32_t encode_impl(rnnt_b200_handle h, const float* feats, const int32_t* lens_T, int32_t B, int32_t T, float* state_h,
                            float* state_c, int32_t use_state_in, float* enc_out, void* stream, int state_ld);
 
@@ -931,18 +999,12 @@ static int32_t encode_impl(rnnt_b200_handle h, const float* feats, const int32_t
   if ((state_h == nullptr) != (state_c == nullptr)) return fail(h, RNNT_B200_ERR_INVALID, "encode: state_h and state_c must both be given");
   cudaStream_t st = (cudaStream_t)stream;
   const int H = c.hidden_sz, X = c.n_mels * c.n_stack, Bp = bp_of(B);
-  // Sub-batch policy (RNNT_SUB32: -1 default, 0 never, 1 always): stateless offline batches run as 32-row sub-batches of the
-  // cluster split-K kernel (measured: 64 utterances 50.0k x real-time vs 44.6k in one 64-row launch of the round-1 kernel, 256
-  // utterances equal); streaming ticks (T = 2, carried state) are faster in one wide launch of the round-1 kernel (8.7k vs 8.0k x)
-  static const int sub32 = [] { const char* e = getenv("RNNT_SUB32"); return e ? atoi(e) : -1; }();
-  static const int lstm_v0 = [] { const char* e = getenv("RNNT_LSTM_V"); return e ? atoi(e) : 2; }();
-  const bool want32 = sub32 == 1 || (sub32 == -1 && !state_h);
-  const int enc_cap = (want32 && lstm_v0 == 2 && h->lstm_tc2_ok) ? 32 : 128;   // the cluster split-K kernel takes 32 rows per launch
-  if (c.gemm_mode == RNNT_B200_GEMM_TC_FP16X3 && h->lstm_tc_ok && B > enc_cap) {
-    // independent utterances / streams: batches beyond the persistent LSTM kernel's capacity run as sub-batches; the state
-    // [L][state_ld][H] is sliced by rows (every layer passes its own base pointer to the kernel)
-    for (int b0 = 0; b0 < B; b0 += enc_cap) {
-      const int nb = std::min(enc_cap, B - b0);
+  const EncoderRoute rt = route_encoder(h, B, state_h != nullptr);
+  if (B > rt.rows) {
+    // independent utterances / streams: the state [L][state_ld][H] is sliced by rows (every layer passes its own base pointer
+    // to the kernel).  Each sub-batch routes again at its own size, so a short last one may take another kernel.
+    for (int b0 = 0; b0 < B; b0 += rt.rows) {
+      const int nb = std::min(rt.rows, B - b0);
       const int r = encode_impl(h, feats + (size_t)b0 * T * X, lens_T ? lens_T + b0 : nullptr, nb, T,
                                 state_h ? state_h + (size_t)b0 * H : nullptr, state_c ? state_c + (size_t)b0 * H : nullptr, use_state_in,
                                 enc_out + (size_t)b0 * T * H, stream, state_ld);
@@ -958,29 +1020,21 @@ static int32_t encode_impl(rnnt_b200_handle h, const float* feats, const int32_t
     const EncLayer& L = h->enc[l];
     const float* A = l == 0 ? h->lnx.as<float>() : ((l - 1) & 1 ? h->yb.as<float>() : h->ya.as<float>());
     float* y = (l == c.enc_layers - 1) ? enc_out : (l & 1 ? h->yb.as<float>() : h->ya.as<float>());
-    const bool tc = c.gemm_mode == RNNT_B200_GEMM_TC_FP16X3;
     if (h->ev) cudaEventRecord(h->ev[6 + 2 * l], st);
-    LstmTcPlan pl;
-    const bool tc_rec = tc && h->lstm_tc_ok && B <= 128 && lstm_tc_plan(H, B, h->sm_count, &pl);
-    static const int lstm_v = [] { const char* e = getenv("RNNT_LSTM_V"); return e ? atoi(e) : 2; }();
-    LstmTc2Plan pl2;
-    const bool tc_rec2 = tc && lstm_v == 2 && h->lstm_tc2_ok && B <= 32 && lstm_tc2_plan(H, B, h->sm_count, &pl2);
-    if (tc) {
+    if (c.gemm_mode == RNNT_B200_GEMM_TC_FP16X3) {
       CK(h->a_img.ensure(gemm_tc_a_image_bytes(M, std::max(L.in, H))));
       // layer 0 reads the LayerNorm output; deeper layers find their operand image already written
       // by the previous layer's recurrent kernel (when that ran on the tensor-core path)
-      if (l == 0 || !(tc_rec || tc_rec2)) LAUNCH(1, launch_to_image(A, L.in, M, L.in, 128, h->a_img.as<uint8_t>(), st));
+      if (l == 0 || rt.kernel == RecKernel::Fp32) LAUNCH(1, launch_to_image(A, L.in, M, L.in, 128, h->a_img.as<uint8_t>(), st));
       LAUNCH(1, launch_gemm_tc(h->a_img.as<uint8_t>(), h->Wih_img[l], L.bias_r, h->xp.as<float>(), 4 * H, M, 4 * H, L.in, st));
     } else {
       LAUNCH(1, launch_gemm_nt_f32(A, L.in, L.Wih_r, L.in, L.bias_r, h->xp.as<float>(), 4 * H, M, 4 * H, L.in, st));
     }
     if (h->ev) cudaEventRecord(h->ev[7 + 2 * l], st);
-    if (tc_rec2) {
+    if (rt.kernel == RecKernel::Tc2) {
       // cluster split-K kernel (lstm_tc2.cu): 4x less operand ingest per step, tagged h exchange
-      const size_t ximg = (size_t)pl2.KB * 8192;
       CK(h->x_img[0].ensure(img_bytes(128, H, 128)));
       CK(h->x_img[1].ensure(img_bytes(128, H, 128)));
-      (void)ximg;
       CK(h->gbar.ensure(1024));
       CK(cudaMemsetAsync(h->gbar.p, 0, 4, st));
       LstmTc2Args a;
@@ -996,65 +1050,19 @@ static int32_t encode_impl(rnnt_b200_handle h, const float* feats, const int32_t
       a.state_c_out = state_c ? state_c + (size_t)l * state_ld * H : nullptr;
       a.barrier = h->gbar.as<unsigned int>();
       a.T = T; a.B = B; a.H = H;
-      static const int dsm_async = [] { const char* e = getenv("RNNT_DSM_ASYNC"); return e ? atoi(e) : 1; }();
-      a.dsm_async = dsm_async;
-      static const int trig = [] { const char* e = getenv("RNNT_TRIG"); return e ? atoi(e) : 3; }();
-      a.trig_lanes = std::max(1, std::min(trig, 8));
-      static const bool dbg_on2 = getenv("RNNT_LSTM_DBG") != nullptr;
-      unsigned long long* dbg = nullptr;
-      unsigned long long* dbg_all = nullptr;
-      if (dbg_on2 && l == 0) {
-        CK(cudaMalloc((void**)&dbg, (size_t)T * 32 + 128));
-        CK(cudaMemset(dbg, 0, (size_t)T * 32 + 128));
-        CK(cudaMalloc((void**)&dbg_all, (size_t)pl2.grid * T * 16));
-        CK(cudaMemset(dbg_all, 0, (size_t)pl2.grid * T * 16));
-        a.dbg = dbg;
-        a.dbg_all = dbg_all;
+      static const bool stamps = getenv("RNNT_LSTM_DBG") != nullptr;
+      if (stamps && l == 0) {
+        CK(cudaMalloc((void**)&a.dbg, (size_t)T * 32 + 128));
+        CK(cudaMemset(a.dbg, 0, (size_t)T * 32 + 128));
+        CK(cudaMalloc((void**)&a.dbg_all, (size_t)rt.tc2.grid * T * 16));
+        CK(cudaMemset(a.dbg_all, 0, (size_t)rt.tc2.grid * T * 16));
       }
-      LAUNCH(1, launch_lstm_layer_tc2(a, pl2, st));
-      if (dbg_all) {
-        std::vector<unsigned long long> ha((size_t)pl2.grid * T * 2);
-        CK(cudaStreamSynchronize(st));
-        CK(cudaMemcpy(ha.data(), dbg_all, ha.size() * 8, cudaMemcpyDeviceToHost));
-        cudaFree(dbg_all);
-        double sp_pub = 0, sp_red = 0, first_to_last = 0;
-        for (int t = 1; t < T; ++t) {
-          unsigned long long mn = ~0ull, mx = 0, mn2 = ~0ull, mx2 = 0;
-          for (int c2 = 0; c2 < pl2.grid; ++c2) {
-            const unsigned long long a0 = ha[((size_t)c2 * T + t) * 2], a1 = ha[((size_t)c2 * T + t) * 2 + 1];
-            mn = std::min(mn, a0); mx = std::max(mx, a0); mn2 = std::min(mn2, a1); mx2 = std::max(mx2, a1);
-          }
-          sp_pub += (double)(mx - mn); sp_red += (double)(mx2 - mn2);
-          unsigned long long pm = 0;
-          for (int c2 = 0; c2 < pl2.grid; ++c2) pm = std::max(pm, ha[((size_t)c2 * T + t - 1) * 2]);
-          first_to_last += (double)(mn2 - pm);   // last publish of step t-1 -> first CTA with complete tiles at step t
-        }
-        fprintf(stderr, "[lstm_tc2 skew] avg ns over %d CTAs: spread of publish times %.0f | spread of tiles-complete times %.0f | last publish(t-1) -> first tiles-complete(t) %.0f\n",
-                pl2.grid, sp_pub / (T - 1), sp_red / (T - 1), first_to_last / (T - 1));
-      }
-      if (dbg) {
-        std::vector<unsigned long long> hb((size_t)T * 4 + 16);
-        CK(cudaStreamSynchronize(st));
-        CK(cudaMemcpy(hb.data(), dbg, (size_t)T * 32 + 128, cudaMemcpyDeviceToHost));
-        cudaFree(dbg);
-        fprintf(stderr, "[lstm_tc2 epilogue cycles/step, CTA 0 thread 0] wait accumulators %.0f | TMEM drain %.0f | scatter issue %.0f | wait tiles %.0f | tile sums %.0f | cell %.0f | publish %.0f | BN outputs %.0f\n",
-                (double)hb[(size_t)T * 4 + 0] / T, (double)hb[(size_t)T * 4 + 1] / T, (double)hb[(size_t)T * 4 + 2] / T, (double)hb[(size_t)T * 4 + 3] / T,
-                (double)hb[(size_t)T * 4 + 4] / T, (double)hb[(size_t)T * 4 + 5] / T, (double)hb[(size_t)T * 4 + 6] / T, (double)hb[(size_t)T * 4 + 7] / T);
-        fprintf(stderr, "[lstm_tc2 loader cycles/step, CTA 0 thread 0] first chunk visible %.0f | k-block 0 valid %.0f | k-blocks 1-3 valid %.0f | stores+fence+arrive %.0f\n",
-                (double)hb[(size_t)T * 4 + 8] / T, (double)hb[(size_t)T * 4 + 9] / T, (double)hb[(size_t)T * 4 + 10] / T, (double)hb[(size_t)T * 4 + 11] / T);
-        double ld = 0, mma = 0, red = 0, fin = 0;
-        for (int t = 1; t < T; ++t) {
-          ld += (double)(hb[t * 4 + 0] - hb[(t - 1) * 4 + 3]);   // previous publish -> K slice of h landed in smem
-          mma += (double)(hb[t * 4 + 1] - hb[t * 4 + 0]);        // -> accumulators ready
-          red += (double)(hb[t * 4 + 2] - hb[t * 4 + 1]);        // TMEM drain + DSMEM scatter + partial tiles complete
-          fin += (double)(hb[t * 4 + 3] - hb[t * 4 + 2]);        // cell + publish
-        }
-        fprintf(stderr, "[lstm_tc2 dbg] B=%d T=%d steps avg ns: publish->h landed %.0f | ->tmem_full %.0f | drain+reduce %.0f | cell+publish %.0f | total/step %.0f\n",
-                B, T, ld / (T - 1), mma / (T - 1), red / (T - 1), fin / (T - 1), (double)(hb[(T - 1) * 4 + 3] - hb[3]) / (T - 1));
-      }
+      LAUNCH(1, launch_lstm_layer_tc2(a, rt.tc2, st));
+      if (a.dbg)
+        if (int r = report_lstm_stamps(h, a, rt.tc2.grid, st)) return r;
       continue;
     }
-    if (tc_rec) {
+    if (rt.kernel == RecKernel::Tc) {
       const size_t ximg = img_bytes(128, H, 128);
       CK(h->x_img[0].ensure(ximg));
       CK(h->x_img[1].ensure(ximg));
@@ -1073,29 +1081,7 @@ static int32_t encode_impl(rnnt_b200_handle h, const float* feats, const int32_t
       a.state_c_out = state_c ? state_c + (size_t)l * state_ld * H : nullptr;
       a.barrier = h->gbar.as<unsigned int>();
       a.T = T; a.B = B; a.H = H;
-      static const bool dbg_on = getenv("RNNT_LSTM_DBG") != nullptr;
-      unsigned long long* dbg = nullptr;
-      if (dbg_on && l == 0) {
-        CK(cudaMalloc((void**)&dbg, (size_t)T * 32));
-        CK(cudaMemset(dbg, 0, (size_t)T * 32));
-        a.dbg = dbg;
-      }
-      LAUNCH(1, launch_lstm_layer_tc(a, pl, st));
-      if (dbg) {
-        std::vector<unsigned long long> hb((size_t)T * 4);
-        CK(cudaStreamSynchronize(st));
-        CK(cudaMemcpy(hb.data(), dbg, (size_t)T * 32, cudaMemcpyDeviceToHost));
-        cudaFree(dbg);
-        double w = 0, ld = 0, mma = 0, epi = 0;
-        for (int t = 1; t < T; ++t) {
-          w += (double)(hb[t * 4 + 0] - hb[(t - 1) * 4 + 3]);   // counter visible after previous arrive
-          ld += (double)(hb[t * 4 + 1] - hb[t * 4 + 0]);        // barrier passed -> last operand stage landed
-          mma += (double)(hb[t * 4 + 2] - hb[t * 4 + 0]);       // barrier passed -> accumulators ready
-          epi += (double)(hb[t * 4 + 3] - hb[t * 4 + 2]);       // epilogue incl. fences and arrive
-        }
-        fprintf(stderr, "[lstm_tc dbg] B=%d T=%d steps avg ns: wait-after-arrive %.0f | barrier->last-stage-landed %.0f | barrier->tmem_full %.0f | epilogue %.0f | total/step %.0f\n",
-                B, T, w / (T - 1), ld / (T - 1), mma / (T - 1), epi / (T - 1), (double)(hb[(T - 1) * 4 + 3] - hb[3]) / (T - 1));
-      }
+      LAUNCH(1, launch_lstm_layer_tc(a, rt.tc, st));
       continue;
     }
     if (use_state_in) {
@@ -1166,6 +1152,66 @@ int32_t rnnt_b200_joint(rnnt_b200_handle h, const float* h_pred, const float* h_
   return RNNT_B200_OK;
 }
 
+struct DecoderRoute {
+  RecKernel kernel;
+  int rows;          // rows per launch: a call with more rows runs as consecutive sub-batches
+  DecodeTcPlan tc;   // plan of a launch of min(B, rows) rows (kernel Tc)
+};
+
+// The decode loop's kernel for a call of B rows; stateful: the call carries predictor state or a registered LM state.  The
+// round-1 kernel takes up to 64 utterances; the cluster kernel 32, and stateless calls beyond that run as 32-row sub-batches
+// of it (same policy as the encoder, see route_encoder).  With a fused language model the loop runs in the round-1 kernel
+// where its LM phases fit the shape, else in the fp32 cooperative kernel (decode.cu), whatever gemm_mode says.
+static DecoderRoute route_decoder(rnnt_b200_handle h, int B, bool stateful) {
+  const rnnt_b200_config& c = h->cfg;
+  DecoderRoute r = {};
+  r.kernel = RecKernel::Fp32;
+  r.rows = kDecodeMaxBatch;
+  const bool tc = c.gemm_mode == RNNT_B200_GEMM_TC_FP16X3 && h->dec_tc_ok && (c.lm_layers == 0 || h->lm_tc_ok);
+  if (tc) {
+    r.rows = 64;
+    if (!stateful && h->dec_tc2_ok) r.rows = 32;   // (only where the round-1 kernel is usable too)
+  }
+  // The predictor state [Lp][state_ld][H] / [B][H] is sliceable by rows (the kernels take the layer stride), the fused LM's
+  // feature-major state blob is not: with a registered LM blob the call runs in one launch, whatever its size.
+  if (h->lm_blob) r.rows = std::max(r.rows, B);
+  const int n = std::min(B, r.rows);
+  if (h->dec_tc2_ok && !h->lm_blob && decode_tc2_plan(c.hidden_sz, c.joint_sz, c.vocab_sz, c.pred_layers, n, h->sm_count, c.lm_layers)) {
+    r.kernel = RecKernel::Tc2;
+  } else if (tc) {
+    if (decode_tc_plan(c.hidden_sz, c.joint_sz, c.vocab_sz, c.pred_layers, n, h->sm_count, &r.tc, c.lm_layers, c.lm_hidden_sz)) {
+      r.kernel = RecKernel::Tc;
+    } else if (!stateful && n > 32 &&
+               decode_tc_plan(c.hidden_sz, c.joint_sz, c.vocab_sz, c.pred_layers, 32, h->sm_count, &r.tc, c.lm_layers, c.lm_hidden_sz)) {
+      // some shapes (e.g. H = 1536: 12 vocabulary rows per epilogue thread at 64) only plan for 32, which still beats the
+      // fp32 kernel
+      r.kernel = RecKernel::Tc;
+      r.rows = 32;
+    }
+  }
+  return r;
+}
+
+// RNNT_DEC_DBG: mean time of each segment of the cluster decode kernel's lock-step, from CTA 0's (time, tag) trail, on
+// stderr (tuning aid: synchronises the stream; frees the trail)
+static int32_t report_decode_stamps(rnnt_b200_handle h, const DecodeTc2Args& t, cudaStream_t st) {
+  const int dcap = t.dbg_cap;
+  std::vector<unsigned long long> hb((size_t)dcap * 2);
+  CK(cudaStreamSynchronize(st));
+  CK(cudaMemcpy(hb.data(), t.dbg, (size_t)dcap * 16, cudaMemcpyDeviceToHost));
+  cudaFree(t.dbg);
+  double sum[8] = {0}; int cnt[8] = {0}; int n = 0;
+  for (int i = 1; i < dcap && hb[2 * i]; ++i, ++n) {
+    const int tag = (int)hb[2 * i + 1];
+    if (tag < 8) { sum[tag] += (double)(hb[2 * i] - hb[2 * i - 2]); cnt[tag]++; }
+  }
+  fprintf(stderr, "[decode_tc2 dbg] B=%d stamps=%d avg ns per segment: ->z published %.0f (n=%d) | ->keys published %.0f | ->table reduced %.0f | rule %.0f | C0 %.0f (n=%d) | C1 %.0f | total %.0f us over %d steps\n",
+          t.B, n, cnt[0] ? sum[0] / cnt[0] : 0, cnt[0], cnt[1] ? sum[1] / cnt[1] : 0, cnt[2] ? sum[2] / cnt[2] : 0,
+          cnt[3] ? sum[3] / cnt[3] : 0, cnt[4] ? sum[4] / cnt[4] : 0, cnt[4], cnt[5] ? sum[5] / cnt[5] : 0,
+          n > 1 ? (double)(hb[2 * n] - hb[2]) / 1e3 : 0.0, cnt[3]);
+  return RNNT_B200_OK;
+}
+
 static int32_t decode_greedy_impl(rnnt_b200_handle h, const float* enc, const int32_t* lens_T, int32_t B, int32_t T,
                                   int32_t max_iters, float* pred_state_h, float* pred_out, int32_t use_state_in,
                                   int32_t* tokens_out, int32_t U_cap, int32_t* ntok_out, double* neg_logp_out,
@@ -1190,48 +1236,23 @@ static int32_t decode_greedy_impl(rnnt_b200_handle h, const float* enc, const in
   if (!enc || !tokens_out || !ntok_out || B < 1 || T < 1 || max_iters < 1 || max_iters > 255)
     return fail(h, RNNT_B200_ERR_INVALID, "decode_greedy: bad arguments");
   if ((int64_t)U_cap < (int64_t)max_iters * T) return fail(h, RNNT_B200_ERR_INVALID, "decode_greedy: U_cap < max_iters*T");
-  {
-    // Utterances are independent: larger batches run as consecutive sub-batches of the kernel's capacity
-    // (64 for the tcgen05 kernel, 256 for the fp32 one).  State tensors are [Lp, B, H], i.e. not sliceable
-    // per sub-batch, so stateful (streaming) calls must fit one launch.
-    // With a fused language model the loop runs in the fp32 cooperative kernel (decode.cu), whatever gemm_mode says.
-    int cap = kDecodeMaxBatch;
-    if (c.gemm_mode == RNNT_B200_GEMM_TC_FP16X3 && h->dec_tc_ok && (c.lm_layers == 0 || h->lm_tc_ok)) {
-      // the tcgen05 kernel takes up to 64 utterances; some shapes (e.g. H = 1536: 12 vocabulary rows per epilogue
-      // thread at 64) only plan for 32, which still beats falling back to the fp32 kernel
-      DecodeTcPlan probe;
-      cap = 64;
-      if (B > 32 && !(pred_state_h || pred_out || use_state_in) &&
-          !decode_tc_plan(c.hidden_sz, c.joint_sz, c.vocab_sz, c.pred_layers, std::min(B, 64), h->sm_count, &probe, c.lm_layers, c.lm_hidden_sz) &&
-          decode_tc_plan(c.hidden_sz, c.joint_sz, c.vocab_sz, c.pred_layers, 32, h->sm_count, &probe, c.lm_layers, c.lm_hidden_sz))
-        cap = 32;
-      static const int sub32d = [] { const char* e = getenv("RNNT_SUB32"); return e ? atoi(e) : -1; }();
-      static const int dec_v0 = [] { const char* e = getenv("RNNT_DEC_V"); return e ? atoi(e) : 2; }();
-      const bool stateless = !(pred_state_h || pred_out || use_state_in || h->lm_blob);
-      if ((sub32d == 1 || (sub32d == -1 && stateless)) && dec_v0 == 2 && h->dec_tc2_ok && !h->lm_blob &&
-          decode_tc2_plan(c.hidden_sz, c.joint_sz, c.vocab_sz, c.pred_layers, 32, h->sm_count, c.lm_layers))
-        cap = 32;   // the cluster split-K decode kernel takes 32 utterances (same policy as the encoder, see rnnt_b200_encode)
+  const bool stateful = pred_state_h || pred_out || use_state_in || h->lm_blob;
+  if (stateful && B > kDecodeMaxBatch)
+    return fail(h, RNNT_B200_ERR_INVALID, "decode_greedy: stateful calls are limited to " + std::to_string(kDecodeMaxBatch) + " streams per call");
+  const DecoderRoute rt = route_decoder(h, B, stateful);
+  if (B > rt.rows) {
+    // utterances / streams are independent; each sub-batch routes again at its own size
+    const int H0 = c.hidden_sz;
+    for (int b0 = 0; b0 < B; b0 += rt.rows) {
+      const int nb = std::min(rt.rows, B - b0);
+      const int r = decode_greedy_impl(h, enc + (size_t)b0 * T * H0, lens_T ? lens_T + b0 : nullptr, nb, T, max_iters,
+                                       pred_state_h ? pred_state_h + (size_t)b0 * H0 : nullptr, pred_out ? pred_out + (size_t)b0 * H0 : nullptr,
+                                       use_state_in, tokens_out + (size_t)b0 * U_cap, U_cap, ntok_out + b0,
+                                       neg_logp_out ? neg_logp_out + b0 : nullptr, iters_out ? iters_out + (size_t)b0 * T : nullptr,
+                                       trace_logp ? trace_logp + (size_t)b0 * trace_cap * c.vocab_sz : nullptr, trace_cap, stream, state_ld);
+      if (r) return r;
     }
-    const bool stateful = pred_state_h || pred_out || use_state_in || h->lm_blob;
-    if (stateful && B > kDecodeMaxBatch)
-      return fail(h, RNNT_B200_ERR_INVALID, "decode_greedy: stateful calls are limited to " + std::to_string(kDecodeMaxBatch) + " streams per call");
-    // The predictor state [Lp][state_ld][H] / [B][H] is sliceable by rows (the kernels take the layer stride), so stateful
-    // (streaming) calls beyond the tcgen05 kernels' capacity run as sub-batches as well; only the fused LM's feature-major state blob
-    // is not sliceable: with a registered LM blob a wide call still falls through to the fp32 cooperative kernel below.
-    const bool tc_path = c.gemm_mode == RNNT_B200_GEMM_TC_FP16X3 && h->dec_tc_ok;
-    if (B > cap && (!stateful || (tc_path && !h->lm_blob))) {
-      const int H0 = c.hidden_sz;
-      for (int b0 = 0; b0 < B; b0 += cap) {
-        const int nb = std::min(cap, B - b0);
-        const int r = decode_greedy_impl(h, enc + (size_t)b0 * T * H0, lens_T ? lens_T + b0 : nullptr, nb, T, max_iters,
-                                         pred_state_h ? pred_state_h + (size_t)b0 * H0 : nullptr, pred_out ? pred_out + (size_t)b0 * H0 : nullptr,
-                                         use_state_in, tokens_out + (size_t)b0 * U_cap, U_cap, ntok_out + b0,
-                                         neg_logp_out ? neg_logp_out + b0 : nullptr, iters_out ? iters_out + (size_t)b0 * T : nullptr,
-                                         trace_logp ? trace_logp + (size_t)b0 * trace_cap * c.vocab_sz : nullptr, trace_cap, stream, state_ld);
-        if (r) return r;
-      }
-      return RNNT_B200_OK;
-    }
+    return RNNT_B200_OK;
   }
   if (use_state_in && (!pred_state_h || !pred_out)) return fail(h, RNNT_B200_ERR_INVALID, "decode_greedy: use_state_in needs pred_state_h and pred_out");
   if (trace_logp && trace_cap < 1) return fail(h, RNNT_B200_ERR_INVALID, "decode_greedy: trace_cap < 1");
@@ -1249,9 +1270,7 @@ static int32_t decode_greedy_impl(rnnt_b200_handle h, const float* enc, const in
     LAUNCH(1, launch_gemm_nt_f32(enc, H, h->W1 + H, 2 * H, h->dw.b1, h->ep.as<float>(), J, M, J, H, st));
   }
   if (h->ev) cudaEventRecord(h->ev[3], st);
-  static const int dec_v = [] { const char* e = getenv("RNNT_DEC_V"); return e ? atoi(e) : 2; }();
-  if (c.gemm_mode == RNNT_B200_GEMM_TC_FP16X3 && dec_v == 2 && h->dec_tc2_ok && !h->lm_blob &&
-      decode_tc2_plan(H, J, c.vocab_sz, c.pred_layers, B, h->sm_count, c.lm_layers)) {
+  if (rt.kernel == RecKernel::Tc2) {
     // cluster split-K decode (decode_tc2.cu): up to 32 utterances per launch
     const size_t one = decode_tc2_image_bytes();
     const int nimg = decode_tc2_images();
@@ -1273,12 +1292,6 @@ static int32_t decode_greedy_impl(rnnt_b200_handle h, const float* enc, const in
     t.w = h->dw;
     t.w1p_img = h->W1p_img2; t.w2_img = h->W2_img2; t.k1_img = h->K1_img2; t.r_img[0] = h->R_img2[0]; t.r_img[1] = h->R_img2[1];
     for (int i = 0; i < nimg; ++i) t.img[i] = h->dimg.as<uint8_t>() + (size_t)(2 * i) * one;
-    static const int n_spec = [] { const char* e = getenv("RNNT_DEC_SPEC"); return e ? atoi(e) : 2; }();
-    t.n_spec = std::max(1, std::min(n_spec, decode_tc2_max_spec()));
-    static const int dec_tune = [] { const char* e = getenv("RNNT_DEC_TUNE"); return e ? atoi(e) : 6; }();
-    t.tune = dec_tune;
-    static const int dec_trig = [] { const char* e = getenv("RNNT_DEC_TRIG"); return e ? atoi(e) : 6; }();
-    t.trig_lanes = std::max(1, std::min(dec_trig, 8));
     t.img_stride = one;
     t.keys = h->dkeys.as<unsigned long long>();
     t.n_eval = reinterpret_cast<int*>(h->dkeys.as<uint8_t>() + decode_tc2_keys_bytes());
@@ -1288,38 +1301,20 @@ static int32_t decode_greedy_impl(rnnt_b200_handle h, const float* enc, const in
     t.tokens = tokens_out; t.U_cap = U_cap; t.ntok = ntok_out; t.neg_logp = neg_logp_out; t.iters = iters_out;
     t.trace = trace_logp; t.trace_cap = trace_logp ? trace_cap : 0;
     t.barrier = h->gbar.as<unsigned int>();
-    static const int dsm_async2 = [] { const char* e = getenv("RNNT_DSM_ASYNC"); return e ? atoi(e) : 1; }();
-    t.dsm_async = dsm_async2;
-    static const bool ddbg2 = getenv("RNNT_DEC_DBG") != nullptr;
-    unsigned long long* dbg = nullptr;
-    const int dcap = 8192;
-    if (ddbg2) {
-      CK(cudaMalloc((void**)&dbg, (size_t)dcap * 16));
-      CK(cudaMemset(dbg, 0, (size_t)dcap * 16));
-      t.dbg = dbg; t.dbg_cap = dcap;
+    static const bool stamps = getenv("RNNT_DEC_DBG") != nullptr;
+    if (stamps) {
+      t.dbg_cap = 8192;
+      CK(cudaMalloc((void**)&t.dbg, (size_t)t.dbg_cap * 16));
+      CK(cudaMemset(t.dbg, 0, (size_t)t.dbg_cap * 16));
     }
     LAUNCH(trace_logp ? 3 : 2, launch_decode_tc2(t, st));
-    if (dbg) {
-      std::vector<unsigned long long> hb((size_t)dcap * 2);
-      CK(cudaStreamSynchronize(st));
-      CK(cudaMemcpy(hb.data(), dbg, (size_t)dcap * 16, cudaMemcpyDeviceToHost));
-      cudaFree(dbg);
-      double sum[8] = {0}; int cnt[8] = {0}; int n = 0;
-      for (int i = 1; i < dcap && hb[2 * i]; ++i, ++n) {
-        const int tag = (int)hb[2 * i + 1];
-        if (tag < 8) { sum[tag] += (double)(hb[2 * i] - hb[2 * i - 2]); cnt[tag]++; }
-      }
-      fprintf(stderr, "[decode_tc2 dbg] B=%d stamps=%d avg ns per segment: ->z published %.0f (n=%d) | ->keys published %.0f | ->table reduced %.0f | rule %.0f | C0 %.0f (n=%d) | C1 %.0f | total %.0f us over %d steps\n",
-              B, n, cnt[0] ? sum[0] / cnt[0] : 0, cnt[0], cnt[1] ? sum[1] / cnt[1] : 0, cnt[2] ? sum[2] / cnt[2] : 0,
-              cnt[3] ? sum[3] / cnt[3] : 0, cnt[4] ? sum[4] / cnt[4] : 0, cnt[4], cnt[5] ? sum[5] / cnt[5] : 0,
-              n > 1 ? (double)(hb[2 * n] - hb[2]) / 1e3 : 0.0, cnt[3]);
-    }
+    if (t.dbg)
+      if (int r = report_decode_stamps(h, t, st)) return r;
     if (h->ev) cudaEventRecord(h->ev[4], st);
     return RNNT_B200_OK;
   }
-  DecodeTcPlan dpl;
-  if (c.gemm_mode == RNNT_B200_GEMM_TC_FP16X3 && h->dec_tc_ok && (c.lm_layers == 0 || h->lm_tc_ok) &&
-      decode_tc_plan(H, J, c.vocab_sz, c.pred_layers, B, h->sm_count, &dpl, c.lm_layers, c.lm_hidden_sz)) {
+  if (rt.kernel == RecKernel::Tc) {
+    const DecodeTcPlan& dpl = rt.tc;
     const size_t one = (size_t)(std::max(H, J) / 64) * 2 * dpl.Bpad8 * 128;
     const int nimg = 4 + 2 * c.pred_layers;
     CK(h->dimg.ensure(one * nimg));
@@ -1388,29 +1383,7 @@ static int32_t decode_greedy_impl(rnnt_b200_handle h, const float* enc, const in
       L.lmstat = reinterpret_cast<double*>(h->lm_stat.as<uint8_t>() + stat_bytes);
       L.fkeys = reinterpret_cast<unsigned long long*>(h->lm_stat.as<uint8_t>() + 2 * stat_bytes);
     }
-    static const bool ddbg = getenv("RNNT_DEC_DBG") != nullptr;
-    unsigned long long* dbg = nullptr;
-    const int dcap = 8192;
-    if (ddbg) {
-      CK(cudaMalloc((void**)&dbg, (size_t)dcap * 16));
-      CK(cudaMemset(dbg, 0, (size_t)dcap * 16));
-      t.dbg = dbg; t.dbg_cap = dcap;
-    }
     LAUNCH(trace_logp ? 3 : 2, launch_decode_tc(t, dpl, st));
-    if (dbg) {
-      std::vector<unsigned long long> hb((size_t)dcap * 2);
-      CK(cudaStreamSynchronize(st));
-      CK(cudaMemcpy(hb.data(), dbg, (size_t)dcap * 16, cudaMemcpyDeviceToHost));
-      cudaFree(dbg);
-      double sum[8] = {0}; int cnt[8] = {0}; int n = 0;
-      for (int i = 1; i < dcap && hb[2 * i]; ++i, ++n) {
-        const int tag = (int)hb[2 * i + 1];
-        if (tag < 8) { sum[tag] += (double)(hb[2 * i] - hb[2 * i - 2]); cnt[tag]++; }
-      }
-      fprintf(stderr, "[decode_tc dbg] B=%d stamps=%d avg ns per segment: A(pp+z)->arrive %.0f (n=%d) | B(logits)->arrive %.0f (n=%d) | grid wait %.0f | R %.0f | gru0 %.0f (n=%d) | gru1 %.0f\n",
-              B, n, cnt[0] ? sum[0] / cnt[0] : 0, cnt[0], cnt[1] ? sum[1] / cnt[1] : 0, cnt[1], cnt[2] ? sum[2] / cnt[2] : 0,
-              cnt[3] ? sum[3] / cnt[3] : 0, cnt[4] ? sum[4] / cnt[4] : 0, cnt[4], cnt[5] ? sum[5] / cnt[5] : 0);
-    }
     if (h->ev) cudaEventRecord(h->ev[4], st);
     return RNNT_B200_OK;
   }
@@ -1593,15 +1566,11 @@ int32_t rnnt_b200_pipeline_submit(rnnt_b200_handle h, const float* audio, int32_
   const rnnt_b200_config& c = h->cfg;
   const int64_t T = num_steps(c, n);
   if (T < 1) return fail(h, RNNT_B200_ERR_INVALID, "pipeline_submit: input shorter than one stacked row");
-  // RNNT_PIPE_PRIO=0: both internal streams at the same priority and cooperative launches kept (the front-end blocks then
-  // compete with the GEMM blocks of the batch ahead); RNNT_PIPE_SAME=1: no overlap at all (front half on the back stream)
-  static const int prio = [] { const char* e = getenv("RNNT_PIPE_PRIO"); return e ? atoi(e) : 1; }();
-  static const int same = [] { const char* e = getenv("RNNT_PIPE_SAME"); return e ? atoi(e) : 0; }();
   if (!h->pipe_front) {
     int lo = 0, hi = 0;
     CK(cudaDeviceGetStreamPriorityRange(&lo, &hi));   // lo = least urgent (numerically greatest), hi = most urgent
     CK(cudaStreamCreateWithPriority(&h->pipe_front, cudaStreamNonBlocking, lo));
-    CK(cudaStreamCreateWithPriority(&h->pipe_back, cudaStreamNonBlocking, prio ? hi : lo));
+    CK(cudaStreamCreateWithPriority(&h->pipe_back, cudaStreamNonBlocking, hi));
     for (auto& ps : h->pipe)
       for (cudaEvent_t* e : {&ps.in_ready, &ps.front_done, &ps.back_done}) CK(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
   }
@@ -1613,7 +1582,7 @@ int32_t rnnt_b200_pipeline_submit(rnnt_b200_handle h, const float* audio, int32_
   CK(s.ntok.ensure((size_t)B * 4));
   CK(s.nlp.ensure((size_t)B * 8));
   CK(h->t_enc.ensure((size_t)B * T * c.hidden_sz * 4));
-  cudaStream_t st = (cudaStream_t)stream, fs = same ? h->pipe_back : h->pipe_front, bs = h->pipe_back;
+  cudaStream_t st = (cudaStream_t)stream, fs = h->pipe_front, bs = h->pipe_back;
   CK(cudaEventRecord(s.in_ready, st));   // the caller's inputs are complete in `stream` order
   CK(cudaStreamWaitEvent(fs, s.in_ready, 0));
   const float* a_dev = audio;
@@ -1637,10 +1606,10 @@ int32_t rnnt_b200_pipeline_submit(rnnt_b200_handle h, const float* audio, int32_
   CK(cudaStreamWaitEvent(bs, s.front_done, 0));
   h->ev = nullptr;   // no stage events on the pipelined path (stages of consecutive batches overlap)
   struct CoopOff {   // plain launches for the persistent kernels while the front end of the next batch may be resident (kernels.h)
-    bool prev, act;
-    explicit CoopOff(bool a) : prev(coop_launch_enabled()), act(a) { if (act) set_coop_launch(false); }
-    ~CoopOff() { if (act) set_coop_launch(prev); }
-  } coop_off(prio != 0 && !same);
+    bool prev;
+    CoopOff() : prev(coop_launch_enabled()) { set_coop_launch(false); }
+    ~CoopOff() { set_coop_launch(prev); }
+  } coop_off;
   if (int r = rnnt_b200_encode(h, s.feats.as<float>(), lens_T, B, (int)T, nullptr, nullptr, 0, h->t_enc.as<float>(), bs)) return r;
   if (int r = rnnt_b200_decode_greedy(h, h->t_enc.as<float>(), lens_T, B, (int)T, max_iters, nullptr, nullptr, 0, s.tokens.as<int32_t>(), U_cap,
                                       s.ntok.as<int32_t>(), s.nlp.as<double>(), nullptr, nullptr, 0, bs))
@@ -2058,15 +2027,13 @@ int32_t rnnt_b200_selftest_gemm(rnnt_b200_handle h, const float* A, const float*
     LAUNCH(1, launch_gemm_nt_f32(A, K, W, K, bias, C, N, M, N, K, st));
     return RNNT_B200_OK;
   }
-  const bool pair = gemm_mode == 3;   // test hook: force the CTA-pair (cta_group::2) kernel
-  if (gemm_mode != RNNT_B200_GEMM_TC_FP16X3 && !pair) return fail(h, RNNT_B200_ERR_INVALID, "selftest_gemm: unknown gemm_mode");
+  if (gemm_mode != RNNT_B200_GEMM_TC_FP16X3) return fail(h, RNNT_B200_ERR_INVALID, "selftest_gemm: unknown gemm_mode");
   void *ai = nullptr, *wi = nullptr;
   CK(cudaMalloc(&ai, gemm_tc_a_image_bytes(M, K)));
   CK(cudaMalloc(&wi, gemm_tc_w_image_bytes(N, K)));
   cudaError_t e = launch_to_image(A, K, M, K, 128, (uint8_t*)ai, st);
   if (e == cudaSuccess) e = launch_to_image(W, K, N, K, 256, (uint8_t*)wi, st);
-  if (e == cudaSuccess) e = pair ? launch_gemm_tc2((uint8_t*)ai, (uint8_t*)wi, bias, C, N, M, N, K, st)
-                                 : launch_gemm_tc_1cta((uint8_t*)ai, (uint8_t*)wi, bias, C, N, M, N, K, st);
+  if (e == cudaSuccess) e = launch_gemm_tc((uint8_t*)ai, (uint8_t*)wi, bias, C, N, M, N, K, st);
   if (e == cudaSuccess) e = cudaStreamSynchronize(st);
   cudaFree(ai);
   cudaFree(wi);

@@ -38,11 +38,6 @@ __device__ __forceinline__ unsigned ld_acquire_u32(const unsigned* p) {
 __device__ __forceinline__ void red_release_add(unsigned* p, unsigned v) {
   asm volatile("red.release.gpu.global.add.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
 }
-__device__ __forceinline__ unsigned long long gtimer() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-  return t;
-}
 __device__ __forceinline__ void fence_proxy_async_global() { asm volatile("fence.proxy.async.global;" ::: "memory"); }
 __device__ __forceinline__ void named_bar_sync(int id, int n) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(n) : "memory"); }
 
@@ -483,10 +478,6 @@ __global__ void __launch_bounds__(DT_THREADS, 1) decode_tc_kernel(DecodeTcArgs p
       return (ph[rr] + kLoInv * ph[NC + rr]) + (pl[rr] + kLoInv * pl[NC + rr]);
     };
     unsigned ebar = 0;   // grid arrivals so far (same count in every CTA)
-    int ndbg = 0;
-    auto stamp = [&](int tag) {   // tuning aid: (time, tag) trail of CTA 0
-      if (p.dbg && cta == 0 && et == 0 && ndbg < p.dbg_cap) { p.dbg[2 * ndbg] = gtimer(); p.dbg[2 * ndbg + 1] = (unsigned long long)tag; ++ndbg; }
-    };
     // The phase counter only ever grows, and "barrier k complete" is tested as counter >= k * G.  That is only sound
     // if no CTA makes its (k+1)-th arrival before barrier k is complete -- otherwise early arrivals stand in for late
     // ones.  A CTA that consumed a gated operand in this phase has waited by data dependence; a CTA that SAT THE PHASE
@@ -774,7 +765,6 @@ __global__ void __launch_bounds__(DT_THREADS, 1) decode_tc_kernel(DecodeTcArgs p
         lm_pending = false;
       }
       grid_arrive(waited_A);
-      stamp(0);
 
       // ---------------- phase B: logits slice + softmax partials ----------------
       if (in_B) {
@@ -837,9 +827,7 @@ __global__ void __launch_bounds__(DT_THREADS, 1) decode_tc_kernel(DecodeTcArgs p
         }
       }
       grid_arrive(in_B);
-      stamp(1);
       grid_wait();   // every CTA's atomicMax has landed
-      stamp(2);
 
       // ---------------- R: greedy rule (models.py:408-437), identical in every CTA ----------------
       {
@@ -956,10 +944,9 @@ __global__ void __launch_bounds__(DT_THREADS, 1) decode_tc_kernel(DecodeTcArgs p
         named_bar_sync(1, 128);
       }
       const bool any_emit = c.flags[0] != 0, any_active = c.flags[1] != 0;
-      stamp(3);
       if (any_emit) {
         const int nph = (LM && Ll > Lp) ? Ll : Lp;
-        for (int i = 0; i < nph; ++i) { layer_phase(i, true); stamp(4 + (i < 3 ? i : 3)); }
+        for (int i = 0; i < nph; ++i) layer_phase(i, true);
         par ^= 1;
         if (LM) { lpar ^= 1; lm_pending = true; }
       }

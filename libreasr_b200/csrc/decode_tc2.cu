@@ -14,8 +14,9 @@
 //     ([h_hi ; h_lo] x W_hi, h_hi x W_lo: the 3xFP16 split of tc_common.cuh), so a GEMM job costs 32 tcgen05.mma and a
 //     CTA ingests 32 KB of activations per job instead of 128 KB.
 //   * Split-K reduction through distributed shared memory: every epilogue warp folds its TMEM lanes and writes the
-//     32-batch partial rows into the owner CTA's shared memory (st.shared::cluster + remote mbarrier arrive); the owner
-//     (rank r owns rows [r R/4, (r+1) R/4) of the cluster's block) sums the four partial tiles and finalises.
+//     32-batch partial rows into the owner CTA's shared memory (st.async, whose bytes complete a transaction count on
+//     the owner's mbarrier); the owner (rank r owns rows [r R/4, (r+1) R/4) of the cluster's block) sums the four partial
+//     tiles and finalises.
 //   * Activations (g, z, BN(h0'), h0', h1') travel as tagged 16-byte chunks (tc2_common.cuh): published with one
 //     st.relaxed.gpu.v4 by the finalising thread group, polled as data by the consumers' loader warps.  The per-step
 //     arg max is exchanged the same way: every CTA publishes one packed (logit, index, tag) key per utterance, every CTA
@@ -52,6 +53,11 @@ constexpr int D2_RP = 24;         // row stride of a partial tile (max rows fina
 constexpr int D2_K = 1024;        // H = J
 
 constexpr int D2_MAXS = 2;        // joint evaluations per utterance and lock-step (speculative look-ahead frames)
+// Look-ahead frames evaluated per lock-step (<= D2_MAXS; measured on a B200: three frames are slower, 7.12 ms per batch).
+constexpr int D2_SPEC = 2;
+// Producers (of 8) of the polled line whose chunk must carry the new tag before a loader warp issues the loads of a
+// K slice (fewer stale chunks to re-read).  Measured on a B200, ms per batch: 6.52 at 1, 6.36-6.39 at 5-7, 6.42 at 8.
+constexpr int D2_TRIG = 6;
 enum { IMG_G = 0, IMG_X = 1, IMG_H0 = 2, IMG_H1 = 3, IMG_Z0 = 4, IMG_N = 4 + D2_MAXS };
 enum { JOB_A = 0, JOB_B = 1, JOB_K1 = 2, JOB_R0 = 3, JOB_R1 = 4 };
 
@@ -101,7 +107,7 @@ __global__ void __launch_bounds__(D2_THREADS, 1) decode_tc2_kernel(DecodeTc2Args
     for (int i = 0; i < 2; ++i) {
       mbar_init(&tfull[i], 1);
       mbar_init(&tempty[i], 128);
-      mbar_init(&pbar[i], p.dsm_async ? 4 : 16);   // async: one arming arrive per epilogue warp; sync: 4 CTAs x 4 warps
+      mbar_init(&pbar[i], 4);    // one arming arrive per epilogue warp
       mbar_init(&pfree[i], 16);
     }
     mbar_init(w2full, 1);
@@ -232,9 +238,9 @@ __global__ void __launch_bounds__(D2_THREADS, 1) decode_tc2_kernel(DecodeTc2Args
       const unsigned j = job++;
       const int ab = (int)(j & 1u);
       const unsigned n = j >> 1;
-      // async mode: every epilogue warp arms a quarter of the job's bytes (4 sources x rp rows x 32 x 4 B in total): the phase
-      // cannot complete before all four warps have entered the job, so no warp can be lapped by the barrier
-      if (p.dsm_async && lane == 0) mbar_arrive_expect_tx(&pbar[ab], (uint32_t)(D2_NB * rp * 4));
+      // every epilogue warp arms a quarter of the job's bytes (4 sources x rp rows x 32 x 4 B in total): the phase cannot
+      // complete before all four warps have entered the job, so no warp can be lapped by the barrier
+      if (lane == 0) mbar_arrive_expect_tx(&pbar[ab], (uint32_t)(D2_NB * rp * 4));
       mbar_wait(&tfull[ab], n & 1u);
       tc_fence_after();
       const int r = (M == 64) ? q * 16 + lane : q * 32 + lane;
@@ -242,8 +248,7 @@ __global__ void __launch_bounds__(D2_THREADS, 1) decode_tc2_kernel(DecodeTc2Args
       const int dst_rank = mine ? r / rp : 0, lrow = mine ? r % rp : 0;
       const uint32_t dst = mapa(P_u32 + (uint32_t)((((ab * D2_CL + rank) * D2_NB) * D2_RP + lrow) * 4), (uint32_t)dst_rank);
       const uint32_t rbar = mapa(smem_u32(&pbar[ab]), (uint32_t)dst_rank);
-      if (p.dsm_async) mbar_wait_cluster_relaxed(&pfree[ab], (n & 1u) ^ 1u);   // the owners have consumed the tiles of job j - 2
-      else mbar_wait_cluster(&pfree[ab], (n & 1u) ^ 1u);
+      mbar_wait_cluster_relaxed(&pfree[ab], (n & 1u) ^ 1u);   // the owners have consumed the tiles of job j - 2
 #pragma unroll
       for (int hf = 0; hf < 2; ++hf) {
         float d0[16], d1[16], d2[16];
@@ -253,36 +258,23 @@ __global__ void __launch_bounds__(D2_THREADS, 1) decode_tc2_kernel(DecodeTc2Args
         tmem_ld16(tc + 64, d2);     // W_lo * h_hi (x 2^11)
         tmem_ld_wait();
         if (mine) {
-          if (p.dsm_async) {
 #pragma unroll
-            for (int b = 0; b < 16; ++b) st_async_f32(dst + (uint32_t)((hf * 16 + b) * D2_RP * 4), fmaf(d1[b] + d2[b], kLoInv, d0[b]), rbar);
-          } else {
-#pragma unroll
-            for (int b = 0; b < 16; ++b) st_cluster_f32(dst + (uint32_t)((hf * 16 + b) * D2_RP * 4), fmaf(d1[b] + d2[b], kLoInv, d0[b]));
-          }
+          for (int b = 0; b < 16; ++b) st_async_f32(dst + (uint32_t)((hf * 16 + b) * D2_RP * 4), fmaf(d1[b] + d2[b], kLoInv, d0[b]), rbar);
         }
       }
       tc_fence_before();
       mbar_arrive(&tempty[ab]);
-      if (!p.dsm_async) {
-        __syncwarp();
-        if (lane < D2_CL) mbar_arrive_cluster(mapa(smem_u32(&pbar[ab]), (uint32_t)lane));
-      }
       return j;
     };
     auto wait_job = [&](unsigned j) -> const float* {
       const int ab = (int)(j & 1u);
-      if (p.dsm_async) mbar_wait(&pbar[ab], (j >> 1) & 1u);
-      else mbar_wait_cluster(&pbar[ab], (j >> 1) & 1u);
+      mbar_wait(&pbar[ab], (j >> 1) & 1u);
       return P + (size_t)((ab * D2_CL) * D2_NB + fb) * D2_RP;   // + src * 32 * 24 ; this thread's batch row
     };
     auto release_job = [&](unsigned j) {
       const int ab = (int)(j & 1u);
       __syncwarp();
-      if (lane < D2_CL) {
-        if (p.dsm_async) mbar_arrive_cluster_relaxed(mapa(smem_u32(&pfree[ab]), (uint32_t)lane));   // (the values read are already consumed: program order suffices)
-        else mbar_arrive_cluster(mapa(smem_u32(&pfree[ab]), (uint32_t)lane));
-      }
+      if (lane < D2_CL) mbar_arrive_cluster_relaxed(mapa(smem_u32(&pfree[ab]), (uint32_t)lane));   // (the values read are already consumed: program order suffices)
     };
     auto sum2 = [&](const float* pr, int off, float* o, int nfl) {   // o[i] = sum over the 4 sources, nfl in {2, 4, 6}
 #pragma unroll
@@ -479,7 +471,6 @@ __global__ void __launch_bounds__(D2_THREADS, 1) decode_tc2_kernel(DecodeTc2Args
           }
         }
         };
-        if (!(p.tune & 2)) second_pass();
         // Arg-max exchange in two hops: every CTA hands its keys to the cluster leader through DSMEM (st.async, 117 ns), the
         // leader folds the four and publishes ONE tagged entry per (frame, utterance pair); every CTA then reads the 32-cluster
         // table of all look-ahead frames in a single pass (8 chunks per thread at two frames).
@@ -515,7 +506,7 @@ __global__ void __launch_bounds__(D2_THREADS, 1) decode_tc2_kernel(DecodeTc2Args
 #pragma unroll
               for (int i = 0; i < 4; ++i) r[zs][i] = ld_relaxed_v4(src + ((size_t)zs * D2_NCL + 8 * i) * D2_NB);
             }
-          if (p.tune & 2) second_pass();   // while the table loads are in flight
+          second_pass();   // while the table loads are in flight
           for (;;) {
             uint32_t bad = 0;
 #pragma unroll
@@ -558,25 +549,21 @@ __global__ void __launch_bounds__(D2_THREADS, 1) decode_tc2_kernel(DecodeTc2Args
       {
         // every thread replays the rule for ITS utterance on the reduced keys (read-only) to learn the token it will emit, and
         // requests that token's table row now: the L2 round trip overlaps warp 0's rule and the barrier behind it
-        if (p.tune & 4) {
-          int tokc = -1;
-          if (bvalid && c.active[fb] != 0) {
-            int tl = c.t[fb];
-            const int ln = c.len[fb];
+        if (bvalid && c.active[fb] != 0) {
+          int tl = c.t[fb];
+          const int ln = c.len[fb];
 #pragma unroll
-            for (int zs = 0; zs < D2_MAXS; ++zs) {
-              if (zs < NS && tokc < 0 && tl < ln) {
-                unsigned long long key = 0ull;
+          for (int zs = 0; zs < D2_MAXS; ++zs) {
+            if (zs < NS && tok_pre < 0 && tl < ln) {
+              unsigned long long key = 0ull;
 #pragma unroll
-                for (int g = 0; g < 8; ++g) key = c.kred[zs][g][fb] > key ? c.kred[zs][g][fb] : key;
-                const int am2 = (int)(0x7FFFFFFFu - (unsigned)((key & 0xFFFFFFFFull) >> 1));
-                if (am2 == w.blank) ++tl; else tokc = am2;
-              }
+              for (int g = 0; g < 8; ++g) key = c.kred[zs][g][fb] > key ? c.kred[zs][g][fb] : key;
+              const int am2 = (int)(0x7FFFFFFFu - (unsigned)((key & 0xFFFFFFFFull) >> 1));
+              if (am2 == w.blank) ++tl; else tok_pre = am2;
             }
           }
-          if (tokc >= 0) load_table0(tokc, vpre);
-          tok_pre = tokc;
         }
+        if (tok_pre >= 0) load_table0(tok_pre, vpre);
         if (et < B) {
           const int bb = et;
           unsigned char emit = 0;
@@ -670,7 +657,7 @@ __global__ void __launch_bounds__(D2_THREADS, 1) decode_tc2_kernel(DecodeTc2Args
       const uint32_t tag = (n >> 1) & 1u;
       const uint8_t* src = img_ptr(img, n) + slice_off + (size_t)lt * 16;
       uint4 r[16];
-      poll_issue<16>(src, 16, tag, r, p.trig_lanes);
+      poll_issue<16>(src, 16, tag, r, D2_TRIG);
 #pragma unroll
       for (int kb = 0; kb < D2_KS; ++kb, ++ga) {
         poll_validate_kb<16>(src, kb, tag, r);
@@ -888,10 +875,11 @@ bool decode_tc2_plan(int H, int J, int V, int Lp, int B, int sms, int lm_layers)
 size_t decode_tc2_image_bytes() { return (size_t)(D2_K / 64) * 8192; }        // one buffer of one activation image
 size_t decode_tc2_keys_bytes() { return (size_t)2 * D2_MAXS * D2_NCL * D2_NB * 8; }
 int decode_tc2_images() { return IMG_N; }
-int decode_tc2_max_spec() { return D2_MAXS; }
 int decode_tc2_part_ctas() { return D2_G; }
 
 cudaError_t launch_decode_tc2(const DecodeTc2Args& a, cudaStream_t st) {
+  DecodeTc2Args args = a;
+  args.n_spec = D2_SPEC;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(D2_G);
   cfg.blockDim = dim3(D2_THREADS);
@@ -906,7 +894,7 @@ cudaError_t launch_decode_tc2(const DecodeTc2Args& a, cudaStream_t st) {
   // cooperative unless switched off (kernels.h: coop_launch_enabled; the plan has verified with
   // cudaOccupancyMaxActiveClusters that all clusters fit)
   cfg.numAttrs = coop_launch_enabled() ? 2 : 1;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, decode_tc2_kernel, a);
+  cudaError_t e = cudaLaunchKernelEx(&cfg, decode_tc2_kernel, args);
   if (e != cudaSuccess) return e;
   return launch_decode_finish(a.part, a.n_eval, a.B, D2_G, D2_NB, a.max_steps, a.neg_logp, a.trace, a.trace_lse, a.trace_cap, a.w.V, st);
 }

@@ -9,8 +9,6 @@
 // samples are non-zero), the CTA then writes the X = n_mels*n_stack floats of the row with
 // one coalesced pass.  Audio is read once per frame (25% of frames are
 // shared by two rows and recomputed: the kernel is FFT-, not HBM-bound; see DESIGN.md).
-#include <cstdlib>
-
 #include "kernels.h"
 
 namespace rnnt {
@@ -206,10 +204,9 @@ size_t frontend_smem_bytes(int n_stack, int n_mels) {
 cudaError_t launch_mel_stack(const FrontendArgs& a, int B, cudaStream_t st) {
   if (a.n_stack > kFrontendMaxWarps) return cudaErrorInvalidValue;
   const size_t smem = frontend_smem_bytes(a.n_stack, a.n_mels);
-  static const int occ = [] { const char* e = getenv("RNNT_FE_OCC"); return e ? atoi(e) : 2; }();
   dim3 grid(a.T_out, B);
   cudaError_t e;
-  if (occ >= 2 && a.n_stack * 32 <= 320) {
+  if (a.n_stack * 32 <= 320) {   // two CTAs per SM
     e = cudaFuncSetAttribute(mel_stack_kernel<320, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     mel_stack_kernel<320, 2><<<grid, a.n_stack * 32, smem, st>>>(a);

@@ -12,8 +12,6 @@
 // 64-deep k-block from the operand images with two TMA bulk copies into a 2-stage ring,
 // one thread of warp 1 issues 12 tcgen05.mma (M128 N256 K16) per k-block into 512 TMEM
 // columns (D0 | D1), warps 2-5 drain TMEM (tcgen05.ld 32x32b) and write C with the bias.
-#include <cstdlib>
-
 #include "kernels.h"
 #include "tc_common.cuh"
 
@@ -184,7 +182,7 @@ cudaError_t configure_gemm_tc() {
   return cudaFuncSetAttribute(gemm_tc_f16x3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GT_SMEM_BYTES);
 }
 
-// an even number of 128-row tiles: the CTA-pair kernel (gemm_tc2.cu) reads row tiles in pairs
+// rounded to an even number of 128-row tiles: the recurrent kernels write their outputs into this image too
 size_t gemm_tc_a_image_bytes(int64_t M, int K) { return img_bytes(round_up(M, 2 * GT_BM), K, GT_BM); }
 size_t gemm_tc_w_image_bytes(int N, int K) { return img_bytes(N, K, GT_BN); }
 
@@ -195,22 +193,14 @@ cudaError_t launch_to_image(const float* src, int ld, int64_t R, int K, int TR, 
   return cudaGetLastError();
 }
 
-cudaError_t launch_gemm_tc_1cta(const uint8_t* a_img, const uint8_t* w_img, const float* bias, float* C, int ldc, int64_t M, int N,
-                                int K, cudaStream_t st) {
+cudaError_t launch_gemm_tc(const uint8_t* a_img, const uint8_t* w_img, const float* bias, float* C, int ldc, int64_t M, int N,
+                           int K, cudaStream_t st) {
   if ((ldc & 3) || (N & 3)) return cudaErrorInvalidValue;
   GemmTcArgs a;
   a.a_img = a_img; a.b_img = w_img; a.bias = bias; a.C = C; a.ldc = ldc; a.M = M; a.N = N; a.KB = (int)ceil_div(K, kImgK);
   dim3 grid((unsigned)ceil_div(N, GT_BN), (unsigned)ceil_div(M, GT_BM));
   gemm_tc_f16x3_kernel<<<grid, GT_THREADS, GT_SMEM_BYTES, st>>>(a);
   return cudaGetLastError();
-}
-
-// The CTA-pair kernel moves a third fewer operand bytes per FLOP; a single 128-row tile has no partner to pair with.
-cudaError_t launch_gemm_tc(const uint8_t* a_img, const uint8_t* w_img, const float* bias, float* C, int ldc, int64_t M, int N,
-                           int K, cudaStream_t st) {
-  static const bool pair = [] { const char* e = getenv("RNNT_GEMM_2CTA"); return e && e[0] == '1'; }();
-  if (pair && M > GT_BM) return launch_gemm_tc2(a_img, w_img, bias, C, ldc, M, N, K, st);
-  return launch_gemm_tc_1cta(a_img, w_img, bias, C, ldc, M, N, K, st);
 }
 
 }  // namespace rnnt

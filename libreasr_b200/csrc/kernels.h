@@ -59,12 +59,6 @@ size_t gemm_tc_w_image_bytes(int N, int K);       // weight operand image, 256-r
 // fp32 row-major [R][ld] -> hi/lo fp16 operand image with TR-row tiles (tc_common.cuh)
 cudaError_t launch_to_image(const float* src, int ld, int64_t R, int K, int TR, uint8_t* img, cudaStream_t st);
 // C[M,N] = A * W^T + bias from operand images (A: TR=128, W: TR=256)
-// gemm_tc2.cu: CTA-pair (cta_group::2) variant, 256 x 256 pair tiles; a_img must hold an even number of 128-row tiles
-cudaError_t configure_gemm_tc2();
-cudaError_t launch_gemm_tc_1cta(const uint8_t* a_img, const uint8_t* w_img, const float* bias, float* C, int ldc, int64_t M, int N, int K,
-                                cudaStream_t st);
-cudaError_t launch_gemm_tc2(const uint8_t* a_img, const uint8_t* w_img, const float* bias, float* C, int ldc, int64_t M, int N, int K,
-                            cudaStream_t st);
 cudaError_t launch_gemm_tc(const uint8_t* a_img, const uint8_t* w_img, const float* bias, float* C, int ldc, int64_t M, int N,
                            int K, cudaStream_t st);
 
@@ -88,7 +82,6 @@ struct LstmTcArgs {
   const float* state_h_in; const float* state_c_in;   // [B][H] or nullptr
   float* state_h_out; float* state_c_out;             // [B][H] or nullptr
   unsigned int* barrier;     // [H/64] per-k-block readiness counters, zero at launch
-  unsigned long long* dbg;   // optional [T][4] globaltimer stamps of CTA 0 (tuning aid), or nullptr
   int T, B, H;
   // filled from the plan by the launcher
   int U, NC, KB, Bpad8, stages, w_resident, bar_offset, tmem_cols, kps, mma_m, fused, pre_offset;
@@ -120,8 +113,6 @@ struct LstmTc2Args {
   unsigned long long* dbg_all;   // optional [grid][T][2] (publish, tiles complete) stamps of every CTA: skew diagnosis
   int T, B, H;
   int KS, KB;                // filled from the plan by the launcher
-  int dsm_async;             // partial tiles through st.async + complete_tx (1) or st.shared::cluster + release arrive (0)
-  int trig_lanes;            // producers (of 8) whose chunk must be visible before the bulk load of a K slice is issued
 };
 cudaError_t configure_lstm_tc2();
 bool lstm_tc2_plan(int H, int B, int sms, LstmTc2Plan* pl);
@@ -277,7 +268,6 @@ struct DecodeTcArgs {
   int state_ld;                    // batch stride of state_h per layer (= B unless the launch is a slice of a larger state)
   int32_t* tokens; int U_cap; int32_t* ntok; double* neg_logp; uint8_t* iters; float* trace; int trace_cap;
   unsigned int* barrier;           // grid phase counter, zero at launch
-  unsigned long long* dbg; int dbg_cap;   // optional (time, tag) trail of CTA 0 (tuning aid)
   // filled from the plan by the launcher
   int Uc, NC_A, NC_B, NC_C, NC_max, Bpad8, Bq, mma_m, kps, stages, pre_offset, ctl_offset, bar_offset, tmem_cols, rec_col0, rec_cols;
   int Ul, NC_L, G_l, lm_col0, lm_offset;
@@ -295,9 +285,7 @@ struct DecodeTc2Args {
   const uint8_t* k1_img;
   const uint8_t* r_img[2];
   uint8_t* img[8];                 // tagged activation images g, BN(h0'), h0', h1', z of look-ahead frame 0, 1, ..: 2 buffers of img_stride bytes each
-  int n_spec;                      // joint evaluations per utterance and lock-step (1 = none speculative)
-  int trig_lanes;                  // producers (of 8) whose chunk must be visible before the bulk load of a K slice is issued (RNNT_DEC_TRIG, default 6: measured 6.52 ms per batch at 1, 6.36-6.39 at 5-7, 6.42 at 8)
-  int tune;                        // bit 1: softmax partials behind the key-table loads; bit 2: table row of the emitted token requested ahead of the rule (RNNT_DEC_TUNE, default 6)
+  int n_spec;                      // joint evaluations per utterance and lock-step (1 = none speculative); set by the launcher
   size_t img_stride;
   unsigned long long* keys;        // [2][128 CTAs][32] packed (logit, index, tag) arg-max keys
   const float* ep;                 // [B][T][J] encoder half of the joint incl. b1
@@ -311,8 +299,7 @@ struct DecodeTc2Args {
   int state_ld;                    // batch stride of state_h per layer
   int32_t* tokens; int U_cap; int32_t* ntok; double* neg_logp; uint8_t* iters; float* trace; int trace_cap;
   unsigned int* barrier;           // launch-start counter, zero at launch
-  unsigned long long* dbg; int dbg_cap;
-  int dsm_async;                   // partial tiles through st.async + complete_tx (1) or st.shared::cluster + release arrive (0)
+  unsigned long long* dbg; int dbg_cap;   // optional (time, tag) trail of CTA 0 (tuning aid)
 };
 cudaError_t configure_decode_tc2();
 bool decode_tc2_plan(int H, int J, int V, int Lp, int B, int sms, int lm_layers);
@@ -320,7 +307,6 @@ size_t decode_tc2_image_bytes();   // one buffer of one activation image
 size_t decode_tc2_keys_bytes();
 int decode_tc2_part_ctas();
 int decode_tc2_images();
-int decode_tc2_max_spec();
 cudaError_t launch_decode_tc2(const DecodeTc2Args& a, cudaStream_t st);
 
 // ---------------- beam.cu (batched RNN-T beam search; algorithm defined by oracle/beam.py) ----------------

@@ -38,11 +38,6 @@ __device__ __forceinline__ unsigned ld_acquire_u32(const unsigned* p) {
   asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
   return v;
 }
-__device__ __forceinline__ unsigned long long gtimer() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-  return t;
-}
 __device__ __forceinline__ void red_release_add(unsigned* p, unsigned v) {
   asm volatile("red.release.gpu.global.add.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
 }
@@ -140,7 +135,6 @@ __global__ void __launch_bounds__(LT_THREADS, 1) lstm_layer_tc_kernel(LstmTcArgs
           ready = __ballot_sync(0xffffffffu, ok);
         }
         fence_proxy_async_global();
-        if (gi == 0 && p.dbg && cta == 0 && lane == 0) p.dbg[t * 4 + 0] = gtimer();
         const int s = g % S;
         const uint32_t ph = (g / S) & 1;
         mbar_wait(&sm.empty[s], ph ^ 1);
@@ -174,7 +168,6 @@ __global__ void __launch_bounds__(LT_THREADS, 1) lstm_layer_tc_kernel(LstmTcArgs
         const uint32_t ph = (g / S) & 1;
         mbar_wait(&sm.full[s], ph);
         tc_fence_after();
-        if (p.dbg && cta == 0 && gi == n_groups - 1 && lane == 0) p.dbg[t * 4 + 1] = gtimer();  // last operand stage landed
         if (elect_one()) {
           uint64_t ad = a_desc0 + (uint64_t)(s * stage_u);
           uint64_t bd = b_desc0 + (uint64_t)(wres ? (uint32_t)(gi * KPS) * wt_u : s * stage_u);
@@ -260,7 +253,6 @@ __global__ void __launch_bounds__(LT_THREADS, 1) lstm_layer_tc_kernel(LstmTcArgs
         if (j < upt && valid) xv[j] = *reinterpret_cast<const float4*>(p.xp + row * (size_t)(4 * H) + (size_t)(unit0 + j) * 4);
       mbar_wait(sm.tfull, t & 1);
       tc_fence_after();
-      if (p.dbg && cta == 0 && et == 0) p.dbg[t * 4 + 2] = gtimer();
       float hy[LT_MAX_U];
       if (fused) {
         // accumulator row r: r < Bpad8 -> hi row of batch r; else lo row of batch r - Bpad8.
@@ -343,10 +335,7 @@ __global__ void __launch_bounds__(LT_THREADS, 1) lstm_layer_tc_kernel(LstmTcArgs
       // the BatchNorm(h_t) outputs for the next layer are written after the release, off the critical path.
       if (valid) store_h(p.x_img[(t + 1) & 1], h);
       named_bar_sync(1, 128);
-      if (et == 0) {
-        red_release_add(my_flag, 1u);
-        if (p.dbg && cta == 0) p.dbg[t * 4 + 3] = gtimer();
-      }
+      if (et == 0) red_release_add(my_flag, 1u);
       if (valid) {
         if (p.y) {
           float* yo = p.y + row * H + unit0;

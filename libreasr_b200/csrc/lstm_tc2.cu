@@ -13,9 +13,9 @@
 //     h_{t-1}: 32 KB instead of 128 KB per step (the grid-wide all-gather of lstm_tc.cu shrinks 4x).
 //   * Split-K reduction: epilogue warp q (TMEM lanes 32q..32q+31 = the gate rows of the 8 units CTA q
 //     finalises) folds the three split products and writes its 32 x 32 fp32 partial tile straight into CTA q's
-//     shared memory (st.shared::cluster), then arrives on CTA q's mbarrier (release.cluster).  Every CTA
-//     sums the 4 partial tiles of its 8 units, adds the hoisted input projection, applies the cell with c
-//     (and h) in registers, and publishes h_t.
+//     shared memory with st.async, whose bytes complete a transaction count on CTA q's mbarrier (no fence on
+//     either side).  Every CTA sums the 4 partial tiles of its 8 units, adds the hoisted input projection,
+//     applies the cell with c (and h) in registers, and publishes h_t.
 //   * h exchange without a flag round trip: h_t is published as 16-byte chunks (8 consecutive units of one
 //     batch row, hi or lo halves, already in the swizzled operand-image order) whose last half carries a
 //     1-bit sequence tag in its LSB (the hi half is tagged BEFORE lo is derived from it, so the pair still
@@ -40,6 +40,9 @@ constexpr int L2_CL = 4;          // CTAs per cluster = K slices
 constexpr int L2_UPC = 8;         // units finalised per CTA
 constexpr int L2_NB = 32;         // batch rows per launch (N tile: 32 hi + 32 lo)
 constexpr int L2_MAX_KS = 4;      // k-blocks (64 k) per K slice
+// Producers (of 8) of the polled line whose chunk must carry the new tag before a loader warp issues the loads of its
+// K slice (measured on a B200: 5 and 6 change nothing against 3).
+constexpr int L2_TRIG = 3;
 
 __global__ void __launch_bounds__(L2_THREADS, 1) lstm_layer_tc2_kernel(LstmTc2Args p) {
   extern __shared__ uint8_t smem_raw[];
@@ -69,7 +72,7 @@ __global__ void __launch_bounds__(L2_THREADS, 1) lstm_layer_tc2_kernel(LstmTc2Ar
     for (int i = 0; i < 2; ++i) {
       mbar_init(&tfull[i], 1);
       mbar_init(&tempty[i], 128);
-      mbar_init(&pbar[i], L2_CL);   // sync mode: one remote arrive per source CTA; async mode: one arming arrive per epilogue warp
+      mbar_init(&pbar[i], 4);   // one arming arrive per epilogue warp
     }
     mbar_init(wfull, 1);
     fence_mbar_init();
@@ -137,9 +140,9 @@ __global__ void __launch_bounds__(L2_THREADS, 1) lstm_layer_tc2_kernel(LstmTc2Ar
         xv0 = xr[0];
         xv1 = xr[1];
       }
-      // async mode: every epilogue warp arms a quarter of the step's bytes, so the phase cannot complete (and the barrier cannot
-      // run a phase ahead of a lagging warp) before all four warps have entered the step
-      if (p.dsm_async && lane == 0) mbar_arrive_expect_tx(&pbar[ab], (uint32_t)(L2_NB * 32 * 4));
+      // every epilogue warp arms a quarter of the step's bytes, so the phase cannot complete (and the barrier cannot run a
+      // phase ahead of a lagging warp) before all four warps have entered the step
+      if (lane == 0) mbar_arrive_expect_tx(&pbar[ab], (uint32_t)(L2_NB * 32 * 4));
       mbar_wait(&tfull[ab], (t >> 1) & 1);
       tc_fence_after();
       if (p.dbg && blockIdx.x == 0 && et == 0) p.dbg[t * 4 + 1] = gtimer();
@@ -155,24 +158,14 @@ __global__ void __launch_bounds__(L2_THREADS, 1) lstm_layer_tc2_kernel(LstmTc2Ar
         mbar_arrive(&tempty[ab]);
         if (prof) { const long long c1 = clock64(); cyc[1] += c1 - c0; c0 = c1; }   // TMEM drain
         // my gate row's 32 batch values -> CTA q's partial tile [ab][src = rank][b][row = lane]
+        // (the bytes are counted on the owner's mbarrier: no fence on either side)
         const uint32_t dst = mapa(P_u32 + (uint32_t)(((ab * L2_CL + rank) * L2_NB) * 128 + lane * 4), (uint32_t)q);
-        if (p.dsm_async) {   // the bytes are counted on the owner's mbarrier: no fence on either side
-          const uint32_t rbar = mapa(smem_u32(&pbar[ab]), (uint32_t)q);
+        const uint32_t rbar = mapa(smem_u32(&pbar[ab]), (uint32_t)q);
 #pragma unroll
-          for (int b = 0; b < 32; ++b) st_async_f32(dst + (uint32_t)b * 128u, fmaf(d1[b] + d2[b], kLoInv, d0[b]), rbar);
-        } else {
-#pragma unroll
-          for (int b = 0; b < 32; ++b) st_cluster_f32(dst + (uint32_t)b * 128u, fmaf(d1[b] + d2[b], kLoInv, d0[b]));
-        }
+        for (int b = 0; b < 32; ++b) st_async_f32(dst + (uint32_t)b * 128u, fmaf(d1[b] + d2[b], kLoInv, d0[b]), rbar);
       }
       if (prof) { const long long c1 = clock64(); cyc[2] += c1 - c0; c0 = c1; }   // scatter issue
-      if (p.dsm_async) {
-        mbar_wait(&pbar[ab], (t >> 1) & 1);
-      } else {
-        __syncwarp();
-        if (lane == 0) mbar_arrive_cluster(mapa(smem_u32(&pbar[ab]), (uint32_t)q));
-        mbar_wait_cluster(&pbar[ab], (t >> 1) & 1);
-      }
+      mbar_wait(&pbar[ab], (t >> 1) & 1);
       if (p.dbg && blockIdx.x == 0 && et == 0) p.dbg[t * 4 + 2] = gtimer();
       if (p.dbg_all && et == 0) p.dbg_all[((size_t)blockIdx.x * T + t) * 2 + 1] = gtimer();
       if (prof) { const long long c1 = clock64(); cyc[3] += c1 - c0; c0 = c1; }   // waiting for the four partial tiles
@@ -247,7 +240,7 @@ __global__ void __launch_bounds__(L2_THREADS, 1) lstm_layer_tc2_kernel(LstmTc2Ar
       const uint8_t* src = p.x_img[t & 1] + slice_off + (size_t)lt * 16;
       uint4 r[L2_MAX_KS * 4];
       long long lc0 = lprof ? clock64() : 0;
-      poll_issue<L2_MAX_KS * 4>(src, NL, tag, r, p.trig_lanes);
+      poll_issue<L2_MAX_KS * 4>(src, NL, tag, r, L2_TRIG);
       if (lprof) { const long long c1 = clock64(); lcyc[0] += c1 - lc0; lc0 = c1; }   // until the first chunk of h_{t-1} shows up
 #pragma unroll
       for (int kb = 0; kb < L2_MAX_KS; ++kb) {

@@ -40,24 +40,6 @@ __device__ __forceinline__ uint32_t mapa(uint32_t smem_addr, uint32_t rank) {
   asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_addr), "r"(rank));
   return r;
 }
-__device__ __forceinline__ void st_cluster_f32(uint32_t addr, float v) {
-  asm volatile("st.shared::cluster.f32 [%0], %1;" ::"r"(addr), "f"(v) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {
-  uint32_t ok;
-  do {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.b32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-  } while (!ok);
-}
 __device__ __forceinline__ void cluster_sync_all() {
   asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
 }

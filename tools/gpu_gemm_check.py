@@ -16,7 +16,7 @@ def main():
         ref = (A.double() @ W.double().t() + b.double())
         scale = float(ref.abs().mean())
         row = {"M": M, "N": N, "K": K}
-        for mode in (0, 1, 3):   # 3 = test hook: CTA-pair (cta_group::2) kernel
+        for mode in (0, 1):
             try:
                 C = eng.selftest_gemm(A, W, b, gemm_mode=mode)
                 torch.cuda.synchronize()

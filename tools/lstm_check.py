@@ -1,11 +1,11 @@
-"""Encoder check + timing for one recurrent-kernel version (run on the GPU box).
+"""Encoder check + timing (run on a GPU).
 
-    RNNT_LSTM_V=2 python tools/lstm_check.py --config cfg2 --B 32 --T 124 --out gpurun_out/enc_v2.npy
-    RNNT_LSTM_V=1 python tools/lstm_check.py ... --out gpurun_out/enc_v1.npy --compare gpurun_out/enc_v2.npy
+    python tools/lstm_check.py --config cfg2 --B 32 --T 124 --out enc_a.npy
+    python tools/lstm_check.py ... --out enc_b.npy --compare enc_a.npy
 
 Feeds seeded random features (not audio: the encoder is what is under test), checks the encoder output and
 final state against the CPU oracle on the first `--oracle-rows` utterances (full size would take minutes) and,
-with --compare, against a saved run of the other kernel version.  Prints encode ms (CUDA events, 10 runs).
+with --compare, against a saved run (for example of another build of the library).  Prints encode ms (CUDA events, 10 runs).
 Test infrastructure (imports oracle/).
 """
 import argparse
@@ -49,7 +49,7 @@ def main():
         lens = torch.tensor([max(1, a.T - 3 * b) for b in range(a.B)], dtype=torch.int32)
     fd = feats.cuda()
     ld = lens.cuda() if lens is not None else None
-    res = {"lstm_v": os.environ.get("RNNT_LSTM_V", "default"), "B": a.B, "T": a.T, "config": a.config}
+    res = {"B": a.B, "T": a.T, "config": a.config}
     enc, st = eng.encode(fd, ld, want_state=True)
     torch.cuda.synchronize()
     enc_c = enc.cpu()

@@ -2,7 +2,7 @@
 stall happened, and a determinism check across repeats of the same input.  STRESS_LIB=<librnnt_b200 build> picks the library.
   STRESS_MODE=offline  (default) bench workload, 32 x 10 s on 8 rotated batches: cluster kernels (STRESS_STAGED=1: stage by stage)
   STRESS_MODE=lm       the same batches with the 4x768 LM fused (round-1 decode kernel with LM)
-  STRESS_MODE=b64      64 x 10 s stateless (32-row sub-batches) and RNNT_SUB32=0 style wide launches are chosen by the env
+  STRESS_MODE=b64      64 x 10 s stateless (32-row sub-batches of the cluster kernels)
   STRESS_MODE=cfg4     128 x 15 s on the 6x1536 shape (round-1 kernels, CTAs sitting phases out)
   STRESS_MODE=pipe     the offline workload through rnnt_b200_pipeline_submit / _collect (STRESS_HOST=1: pinned host inputs)
   STRESS_MODE=stream   STRESS_STREAMS (64: round-1 kernels, 32: cluster kernels) concurrent streams through rnnt_b200_stream_push"""
